@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 3
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...        # the reference arm: CPU oracle, all host threads
+    python bench.py ... --dump-outputs DIR      # also write what the last timed step returned, DIR/<name>.npy
 
 A "step" is one pass of the hot path over the resident workload — ONE kernel launch per rank:
 K1 reward9 (Form D, 36 B/eval) with the K2 detect6 corpus scan on its spare warp; the last CTA
@@ -102,6 +103,24 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(out_dir: str, res) -> None:
+    """What a caller of the timed step receives (its ScoreResult: scores, counts, top-K, corpus report; not the timings) as
+    float64 arrays in out_dir/<name>.npy.  The workload comes from SEED, so two builds run with the same arguments can be
+    compared output for output.  Integers are exact in float64 here: counts are at most the record count, indices below it."""
+    os.makedirs(out_dir, exist_ok=True)
+    rep = res.report
+    arrays = {
+        "scores": res.scores, "counts": res.counts, "topk": res.topk,
+        "report_totals": [rep.total, rep.good, rep.bad, rep.none, rep.goodRate, rep.withReward, rep.rewardSum, rep.avgReward,
+                          rep.toolCalls, rep.toolSucc, rep.toolFail, rep.toolSuccessRate],
+        "report_by_mode": [[*rep.byMode[m], rep.byModeGoodRate[m]] for m in range(len(rep.byMode))],
+        "report_dims": [[d.sum, d.count, d.avg, d.low_flag, d.low_severity, d.sugg_flag, d.sugg_priority] for d in rep.dim],
+        "report_patterns": [[p.count, p.flag, p.severity, *p.examples] for p in rep.pat],
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def bind_to_gpu_numa_node(local: int) -> str:
@@ -435,7 +454,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the weak-scaling, compact-layout and e2e legs")
     ap.add_argument("--parity-budget", type=float, default=25.0, help="seconds of oracle time for the full-axis parity check")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the scores, counts, top-K and corpus report of the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; the reference arm scores a different sample")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -470,6 +495,8 @@ def main():
     ms, res, (w0, w1) = H.timed(step, args.steps, args.warmup, sampler)
     clocks = sampler.stop(w0, w1) if rank == 0 else None
     r = res[-1]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r)
     k1 = float(np.mean([x.timing.reward_ms for x in res]))
     launches = int(sum(x.timing.launches for x in res))
     join_wait = float(np.mean([x.timing.join_wait_ms for x in res]))

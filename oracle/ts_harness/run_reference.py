@@ -39,6 +39,9 @@ import minijs as js  # noqa: E402
 TCS_REL = "src/vs/workbench/contrib/senweaver/common/traceCollectorService.ts"
 APO_REL = "src/vs/workbench/contrib/senweaver/common/apoService.ts"
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+# The senweaver-ide checkout the fixtures and ts/patches were generated against (its source is never copied into this
+# repository); SENWEAVER_IDE_CHECKOUT names another.  The tests that need it skip where it is absent.
+CHECKOUT = os.environ.get("SENWEAVER_IDE_CHECKOUT", "/root/reference")
 
 
 # ------------------------------------------------------------------------------------------------ method extraction
@@ -302,7 +305,7 @@ def build_fixtures(ref_root: str):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--reference", default="/root/reference")
+    ap.add_argument("--reference", default=CHECKOUT)
     ap.add_argument("--check", action="store_true", help="compare with the committed fixtures instead of writing them")
     args = ap.parse_args()
     reward, report = build_fixtures(args.reference)

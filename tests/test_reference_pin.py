@@ -24,7 +24,8 @@ sys.path.insert(0, HARNESS)
 import run_reference as rr  # noqa: E402
 from oracle import ts_transcription as ts  # noqa: E402
 
-REF_PRESENT = os.path.exists(os.path.join("/root/reference", rr.TCS_REL))
+REF = rr.CHECKOUT
+REF_PRESENT = os.path.exists(os.path.join(REF, rr.TCS_REL))
 DIMS = ts.DIM_ORDER
 PAT_DESCR = [
     "Users give negative feedback after errors occur in conversations",
@@ -78,8 +79,9 @@ def test_fixtures_come_from_the_reference_text(ref_reward, ref_report):
         return
     import hashlib
     for rel, sha in prov["reference"].items():                                     # the very files they were generated from
-        assert hashlib.sha256(open(os.path.join("/root/reference", rel), "rb").read()).hexdigest() == sha
-    r = subprocess.run([sys.executable, os.path.join(HARNESS, "run_reference.py"), "--check"], capture_output=True, text=True, timeout=600)
+        assert hashlib.sha256(open(os.path.join(REF, rel), "rb").read()).hexdigest() == sha
+    r = subprocess.run([sys.executable, os.path.join(HARNESS, "run_reference.py"), "--reference", REF, "--check"],
+                       capture_output=True, text=True, timeout=600)
     assert r.returncode == 0 and r.stdout.count("identical to what the reference text produces") == 3, r.stdout + r.stderr
 
 

@@ -5,7 +5,9 @@
 Everything they return must equal what the UNPATCHED reference returned for the same inputs (tests/golden/ref_*.json, the parity
 pin): the per-trace reward dimensions and finalReward bit for bit, the whole PromptEffectivenessReport object (tallies, per-mode
 stats in first-appearance order, the six patterns with ids / severities / example previews, the dimension-low patterns, every
-generated suggestion), and the collector / APO stats.  Needs the reference checkout (the patches apply to it)."""
+generated suggestion), and the collector / APO stats.  Those tests need the senweaver-ide checkout (the patches apply to it;
+its source is not part of this repository, see run_reference.CHECKOUT).  The micro-batching test of ts/apoScoringMainService.ts
+needs only this repository."""
 import json
 import math
 import os
@@ -14,9 +16,12 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "src/vs/workbench/contrib/senweaver/common/apoService.ts")),
-                                reason="reference checkout not present")
+sys.path.insert(0, os.path.join(ROOT, "oracle", "ts_harness"))
+import run_reference as rr  # noqa: E402
+
+REF = rr.CHECKOUT
+needs_checkout = pytest.mark.skipif(not os.path.exists(os.path.join(REF, rr.APO_REL)),
+                                    reason="needs the senweaver-ide checkout (SENWEAVER_IDE_CHECKOUT)")
 
 
 def num(v):
@@ -53,6 +58,7 @@ def outputs(orc):
     return rp.build_outputs(REF)
 
 
+@needs_checkout
 def test_the_patched_methods_are_the_ones_that_ran(outputs):
     _, _, calls, lines = outputs
     assert calls["rewardBatch"] > 431 and calls["score"] > 11          # every reward and every report went through the service
@@ -66,6 +72,7 @@ def test_the_patched_methods_are_the_ones_that_ran(outputs):
     assert "R.patterns.forEach" in "\n".join(apo[a - 1:b])
 
 
+@needs_checkout
 def test_patched_reward_signals_equal_the_reference_bit_for_bit(outputs):
     cases = outputs[0]
     want = json.load(open(os.path.join(ROOT, "tests", "golden", "ref_reward_cases.json")))["cases"]
@@ -74,6 +81,7 @@ def test_patched_reward_signals_equal_the_reference_bit_for_bit(outputs):
         assert c["name"] == w["name"] and c["dims"] == w["dims"] and c["finalReward"] == w["finalReward"], c["name"]
 
 
+@needs_checkout
 def test_patched_reports_and_stats_equal_the_reference(outputs):
     reports = outputs[1]
     want = json.load(open(os.path.join(ROOT, "tests", "golden", "ref_report_cases.json")))["corpora"]
@@ -87,6 +95,7 @@ def test_patched_reports_and_stats_equal_the_reference(outputs):
         same(got["stats"], w["stats"], 1e-12, f"{cname}/stats")
 
 
+@needs_checkout
 def test_patched_evaluate_beam_feeds_the_strict_greater_adoption(orc):
     """`_evaluateBeam` (new) + `_applyBeamUpdate` (the reference's inline bookkeeping of APO:1138-1166, moved into a method by the
     patch): scores and top-K come back as little-endian blocks, the beam is the candidates in top-K order with their scores, a new

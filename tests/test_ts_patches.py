@@ -18,7 +18,10 @@ PATCHES = os.path.join(ROOT, "ts", "patches")
 sys.path.insert(0, PATCHES)
 import make_patches as mp  # noqa: E402
 
-REF = "/root/reference"
+sys.path.insert(0, os.path.join(ROOT, "oracle", "ts_harness"))
+import run_reference as rr  # noqa: E402
+
+REF = rr.CHECKOUT
 REF_PRESENT = os.path.exists(os.path.join(REF, mp.TCS))
 # 1-based inclusive line ranges of the reference that no patch may touch
 PROTECTED = {
@@ -68,7 +71,7 @@ def test_new_ts_files_declare_the_channel_and_the_codec():
     assert "export const EMPTY_DIMS" in codec and "export function decodeCorpusReport" in codec
 
 
-@pytest.mark.skipif(not REF_PRESENT, reason="needs the reference checkout")
+@pytest.mark.skipif(not REF_PRESENT, reason="needs the senweaver-ide checkout (SENWEAVER_IDE_CHECKOUT)")
 @pytest.mark.parametrize("rel,_fn,out", mp.TARGETS)
 def test_patches_apply_and_keep_the_interfaces_byte_for_byte(tmp_path, rel, _fn, out):
     src = os.path.join(REF, rel)
